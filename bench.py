@@ -17,6 +17,12 @@ library's default calling convention, reference accl.cpp:780-826).
 `--impl reference` reports why the reference cannot run here; `--impl nccl`
 measures torch.distributed/NCCL on the same buffers sizes for comparison.
 The reference's own sweep benchmark is test/host/xrt/src/bench.cpp:25-61.
+
+`--dump-outputs DIR` writes, after the timed steps, the all-reduce result of
+the last step as DIR/allreduce_out.npy (rank 0; float32, float64 for float64
+runs).  Results larger than DUMP_MAX_ELEMS are sampled at positions drawn from
+a fixed seed.  The operands are seeded too, so two builds run with the same
+arguments can be compared output for output.
 """
 import argparse
 import json
@@ -30,6 +36,22 @@ sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 
 def busbw_factor(p):
     return 2.0 * (p - 1) / p if p > 1 else 1.0
+
+
+DUMP_MAX_ELEMS = 4 << 20  # 16 MiB as float32, 32 MiB as float64
+
+
+def dump_output(out_dir, name, t):
+    """Write the 1-D result `t` (or a seeded sample of it) as out_dir/<name>.npy in float32 / float64."""
+    import numpy as np
+    import torch
+    if t.numel() > DUMP_MAX_ELEMS:
+        g = torch.Generator().manual_seed(0)
+        idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMS,), generator=g).sort().values
+        t = t[idx.to(t.device)]
+    t = t.to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 class ClockSampler:
@@ -88,7 +110,11 @@ def main():
     ap.add_argument("--tune", default="", help="name=value,... runtime knobs (Accl.set_tuning), identical on every rank")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-nccl", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the result of the last timed step to DIR/allreduce_out.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     if args.impl == "reference":
         print(json.dumps({"impl": "reference", "unavailable":
@@ -151,6 +177,8 @@ def main():
         if sampler:
             sampler.start()
         ms = timed(fn, K, W)
+        if args.dump_outputs and rank == 0:
+            dump_output(args.dump_outputs, "allreduce_out", x)
         launches = K
         impl_name = "nccl"
         e2e = None
@@ -189,6 +217,9 @@ def main():
         if sampler:
             sampler.start()
         ms = timed(fn, K, W)
+        if args.dump_outputs and rank == 0:
+            # before the e2e pass below, which writes dst
+            dump_output(args.dump_outputs, "allreduce_out", dst.dev)
         # kernels of this library launched inside the timed region: one k_call per all-reduce (direct launch), or one
         # k_submit proxy per all-reduce handing the command to the resident k_engine kernel (engine mode)
         launches = K

@@ -16,6 +16,10 @@ if "TORCHELASTIC_RUN_ID" in os.environ:   # under torchrun the agent already hos
     dist.init_process_group("accl", init_method="env://", rank=rank, world_size=world)
 else:
     dist.init_process_group("accl", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world)
+if not use_cuda:
+    # emulator ranks are separate processes that can reach a collective more than the engine's default receive
+    # timeout (1 s) apart on a busy host: give them the budget the CUDA backend has by default (32 s)
+    accl_b200.parallel.process_group._primary["accl"].set_timeout(32_000_000)
 t = torch.full((1000,), float(rank + 1))
 dist.all_reduce(t)
 assert torch.all(t == world * (world + 1) / 2), t[:4]

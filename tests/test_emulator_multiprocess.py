@@ -107,8 +107,8 @@ def test_data_parallel_mlp_trains(zero):
     """End-to-end consumer: DDP / ZeRO-1 training of a small MLP, one emulator process per rank."""
     import json
     r = subprocess.run([sys.executable, "-m", "accl_b200.models.emulator", "-n", "2", "--", sys.executable, "-m",
-                        "accl_b200.models.dp_mlp", "--zero", str(zero), "--steps", "20"], cwd=ROOT, capture_output=True,
-                       text=True, timeout=240)
+                        "accl_b200.models.dp_mlp", "--backend", "emulator", "--zero", str(zero), "--steps", "20"], cwd=ROOT,
+                       capture_output=True, text=True, timeout=240)
     assert r.returncode == 0, r.stdout + r.stderr
     line = [l for l in r.stdout.splitlines() if l.startswith("{")][0]
     out = json.loads(line)
@@ -142,7 +142,8 @@ def test_torch_distributed_backend(world, one_hop):
     """`dist.init_process_group("accl")`: all_reduce / broadcast / all_gather / reduce_scatter / all_to_all /
     reduce / send / recv / barrier and DistributedDataParallel through the standard torch.distributed API."""
     import random
-    env = dict(os.environ, PG_PORT=str(random.randint(20000, 40000)), ACCL_EMU_ONE_HOP=one_hop)
+    # no GPU visible: the backend picks the CUDA path whenever it can (test_cuda_engine.py covers that one)
+    env = dict(os.environ, PG_PORT=str(random.randint(20000, 40000)), ACCL_EMU_ONE_HOP=one_hop, CUDA_VISIBLE_DEVICES="")
     r = subprocess.run([sys.executable, "-m", "accl_b200.models.emulator", "-n", str(world), "--", sys.executable,
                         os.path.join(ROOT, "tests", "helpers", "pg_worker.py")], cwd=ROOT, env=env, capture_output=True,
                        text=True, timeout=300)
