@@ -485,8 +485,9 @@ def cuda_world(devices, heap_mb=256, multicast=True, max_ctas=8, engine=False, n
     appear several times: ranks then share that GPU, without NVLS).  `extra`: engine_workers, engine_idle_us,
     stage_kb, ll_kb and every `set_tuning` knob."""
     _prepare_cuda_env()
-    impls = _C.make_cuda_world(list(devices), heap_mb, multicast, max_ctas, engine, nvls_min_ranks, oneshot_kb, nvls_ops,
-                               {k: int(v) for k, v in extra.items()})
+    options = dict(extra, heap_mb=heap_mb, multicast=multicast, max_ctas=max_ctas, engine=engine,
+                   nvls_min_ranks=nvls_min_ranks, oneshot_kb=oneshot_kb, nvls_ops=nvls_ops)
+    impls = _C.make_cuda_world(list(devices), {k: int(v) for k, v in options.items()})
     return [Accl(a, r, len(devices), cuda_device=devices[r]) for r, a in enumerate(impls)]
 
 
@@ -522,8 +523,9 @@ def cuda_rank(rank=None, world_size=None, device=None, addr=None, port=None, hea
         port = int(os.environ.get("ACCL_PORT", int(os.environ.get("MASTER_PORT", 29500)) + 137))
     if os.environ.get("ACCL_BIND_NUMA", "1") != "0":
         bind_to_gpu_numa_node(device)
-    impl = _C.make_cuda_rank(rank, world_size, device, addr, port, heap_mb, multicast, max_ctas, engine,
-                             nvls_min_ranks, oneshot_kb, nvls_ops, {k: int(v) for k, v in extra.items()})
+    options = dict(extra, heap_mb=heap_mb, multicast=multicast, max_ctas=max_ctas, engine=engine,
+                   nvls_min_ranks=nvls_min_ranks, oneshot_kb=oneshot_kb, nvls_ops=nvls_ops)
+    impl = _C.make_cuda_rank(rank, world_size, device, addr, port, {k: int(v) for k, v in options.items()})
     return Accl(impl, rank, world_size, cuda_device=device)
 
 

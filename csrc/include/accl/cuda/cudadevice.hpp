@@ -53,7 +53,19 @@ struct CudaConfig {
   size_t ll_oneshot_max = 32u << 10; // all-reduce: one hop (everybody sends everything) up to this size
   size_t wire_min_bytes = 256u << 10; // compressed-wire collectives from this size on use the fused two-shot
   Tune tune{0, 4, 0, 0, 0, {0, 0, 0}};
+  bool stream_loopback = true; // every stream id is served by FIFO 0 (the reference's loopback user kernel)
 };
+
+// The backend's options by name (construction arguments, Accl.set_tuning, ACCL_TUNE), defined by one table in
+// cudadevice.cpp.  Applies `value` to `c` with the option's unit scaling (`*_kb`, `heap_mb`) and clamp.  `running`:
+// the device already exists, so only the options that may change after construction are accepted.  Returns false
+// for a name that is not accepted.
+bool set_option(CudaConfig &c, const std::string &name, long value, bool running);
+
+// What the planner (plan.hpp) is told about a device: its options plus the geometry it found at construction.
+// `engine_workers`: worker CTAs of the persistent engine, which are the channels of its calls (0: direct launches).
+PlanCfg make_plan_cfg(const CudaConfig &c, bool has_mc, uint32_t heap_world, size_t stg_bytes, size_t ll_bytes,
+                      uint32_t engine_workers);
 
 class CudaDevice;
 
@@ -112,8 +124,9 @@ public:
   RangeAllocator &allocator() { return *alloc_; }
   HostCompletion *host_completions() { return hc_host_; }
   struct PlanCfg plan_cfg() const;
-  // runtime tuning knobs ("hybrid_16ths", "nvls_unroll", "reduce_push", "bcast_flags", "nvls_ctas", "ll_max_bytes",
-  // "ll_oneshot_max", "max_ctas"); must be set identically on every rank.  Returns false for an unknown name.
+  // the options that may change after construction (see set_option); must be set identically on every rank.
+  // set_tuning returns false for a name it does not accept; get_tuning returns -1 for one it does not know, and also
+  // reports the staging sizes "stage_bytes" / "ll_bytes".
   bool set_tuning(const std::string &name, long value);
   long get_tuning(const std::string &name) const;
   // wait until every call started so far has completed (engine quiesce before direct launches share its channels)
@@ -124,7 +137,7 @@ public:
   class Engine *engine() { return engine_.get(); }
   void *plugin_scratch(size_t bytes); // zero-initialised device memory for plugin kernels (grown on demand)
   // FIFO a stream id is served by: the id itself, or 0 while every id loops back through one FIFO (default)
-  uint32_t stream_port_id(uint32_t id) const { return strm_loopback_ ? 0u : id; }
+  uint32_t stream_port_id(uint32_t id) const { return cfg_.stream_loopback ? 0u : id; }
 
 private:
   uint32_t host_config(const CallDesc &d);
@@ -132,7 +145,6 @@ private:
   void sync_ctrl_word(uint32_t byte_off);
   void apply_env_tuning();
   void drain_locked();
-  bool strm_loopback_ = true; // every stream id is served by FIFO 0 (the reference's loopback user kernel)
 
   std::shared_ptr<Oob> oob_;
   CudaConfig cfg_;

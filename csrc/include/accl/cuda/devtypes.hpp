@@ -175,7 +175,7 @@ struct DevWorld {
   uint64_t scr_bytes;
 };
 
-// tuning knobs that travel with every call (set from CudaConfig / ACCL_TUNE_* / Accl.set_tuning)
+// tuning knobs that travel with every call (set from CudaConfig / ACCL_TUNE="name=value,..." / Accl.set_tuning)
 struct Tune {
   uint8_t hybrid_16ths;  // large NVLS all-reduce: 16ths of every shard handled by the peer two-shot body instead
   uint8_t nvls_unroll;   // 16-byte multimem accesses in flight per thread: 2, 4 (default), 8 or 16

@@ -3,6 +3,7 @@
 #include <pybind11/pybind11.h>
 #include <pybind11/stl.h>
 
+#include <algorithm>
 #include <map>
 
 #include "accl/accl.hpp"
@@ -16,125 +17,93 @@ namespace py = pybind11;
 namespace accl {
 namespace cuda {
 
-using Extra = std::map<std::string, long>;
+using OptionMap = std::map<std::string, long>;
 
-static CudaConfig make_cfg(int device, size_t heap_mb, bool multicast, int max_ctas, bool engine, int nvls_min_ranks,
-                           size_t oneshot_kb, int nvls_ops, const Extra &extra) {
+static CudaConfig config_from(const OptionMap &options) {
   CudaConfig c;
-  auto get = [&](const char *k, long dflt) {
-    auto it = extra.find(k);
-    return it == extra.end() ? dflt : it->second;
-  };
-  c.engine_workers = static_cast<int>(get("engine_workers", c.engine_workers));
-  c.engine_idle_us = static_cast<int>(get("engine_idle_us", c.engine_idle_us));
-  c.stage_bytes = static_cast<size_t>(get("stage_kb", 0)) << 10;
-  c.ll_bytes = static_cast<size_t>(get("ll_kb", 0)) << 10;
-  c.host_pipeline_chunk = static_cast<size_t>(get("host_pipeline_chunk_kb", static_cast<long>(c.host_pipeline_chunk >> 10))) << 10;
-  c.device = device;
-  c.heap_bytes = heap_mb << 20;
-  c.multicast = multicast;
-  c.max_ctas = max_ctas;
-  c.engine = engine;
-  c.nvls_min_ranks = nvls_min_ranks;
-  c.oneshot_max_bytes = oneshot_kb << 10;
-  if (nvls_ops >= 0) c.nvls_ops = static_cast<uint32_t>(nvls_ops);
+  for (auto &kv : options)
+    if (!set_option(c, kv.first, kv.second, false)) throw std::invalid_argument("unknown CUDA backend option '" + kv.first + "'");
   return c;
 }
 
-// knobs that are not construction parameters go through set_tuning
-static void apply_extra(CudaDevice &d, const Extra &extra) {
-  for (auto &kv : extra) {
-    if (kv.first == "engine_workers" || kv.first == "engine_idle_us" || kv.first == "stage_kb" || kv.first == "ll_kb" ||
-        kv.first == "host_pipeline_chunk_kb")
-      continue;
-    if (!d.set_tuning(kv.first, kv.second)) throw std::invalid_argument("unknown CUDA backend option '" + kv.first + "'");
-  }
+static CudaDevice *cuda_device(ACCL &a) {
+  auto *d = dynamic_cast<CudaDevice *>(a.device());
+  if (!d) throw std::runtime_error("not a CUDA backend");
+  return d;
+}
+
+static py::dict plan_dict(const WorkItem &w) {
+  static const char *names[] = {"auto", "local", "eager", "nvls", "p2p", "p2p_oneshot", "ll", "staged", "wire"};
+  py::dict d;
+  d["algo"] = w.algo < 9 ? names[w.algo] : "?";
+  d["n_ctas"] = w.n_ctas;
+  d["use_mc"] = (w.flags & WF_USE_MC) != 0;
+  d["oneshot"] = (w.flags & WF_ONESHOT) != 0;
+  return d;
 }
 
 void bind_cuda(py::module_ &m) {
   m.def("cuda_driver_available", [] { return DriverApi::available(); });
   // The call planner (plan.hpp) as a pure function, for unit tests on machines without a GPU: which protocol /
-  // algorithm / channel count a call of `count` elements of `dtype` gets on a communicator of `world` ranks.
-  m.def("cuda_plan", [](operation op, uint32_t count, dataType dtype, uint32_t world, uint32_t max_eager_bytes, uint32_t max_ctas,
-                        bool has_mc, uint32_t nvls_min_ranks, uint64_t oneshot_max_bytes, bool compressed, uint32_t stage_kb,
-                        uint32_t ll_kb, uint32_t ll_max_bytes, uint32_t ll_oneshot_max, uint32_t staged_max_bytes, bool engine_mode) {
+  // algorithm / channel count a call of `count` elements of `dtype` gets on `world` ranks, given the eager limits (default
+  // 64 KiB), the staging regions (1 MiB, LL 256 KiB), and any backend options (CudaConfig defaults otherwise).
+  m.def("cuda_plan", [](operation op, uint32_t count, dataType dtype, uint32_t world, uint32_t max_eager_bytes,
+                        uint32_t eager_rx_buf_bytes, bool has_mc, uint32_t stage_kb, uint32_t ll_kb, bool engine_mode,
+                        bool compressed, const py::kwargs &options) {
+    const CudaConfig cfg = config_from(options.cast<OptionMap>());
     std::vector<uint32_t> exch(exchmem::SIZE_WORDS, 0);
     exch[exchmem::MAX_EAGER_SIZE / 4] = max_eager_bytes;
-    exch[exchmem::EAGER_RX_BUF_SIZE / 4] = 64u << 10;
-    PlanCfg cfg{};
-    cfg.max_ctas = max_ctas;
-    cfg.nvls_min_ranks = nvls_min_ranks;
-    cfg.has_mc = has_mc ? 1 : 0;
-    cfg.heap_world = world;
-    cfg.oneshot_max_bytes = oneshot_max_bytes;
-    cfg.nvls_ops = NVLS_OPS_DEFAULT;
-    cfg.nvls_ctas = 32;
-    cfg.stg_bytes = stage_kb << 10;
-    cfg.ll_bytes = ll_kb << 10;
-    cfg.ll_max_bytes = ll_max_bytes;
-    cfg.ll_oneshot_max = ll_oneshot_max;
-    cfg.staged_max_bytes = staged_max_bytes;
-    cfg.engine_mode = engine_mode ? 1 : 0;
+    exch[exchmem::EAGER_RX_BUF_SIZE / 4] = eager_rx_buf_bytes;
+    // the worker CTAs an engine would start (engine.cu), without its cap by the SM count
+    const uint32_t workers = static_cast<uint32_t>(std::max(1, cfg.engine_workers > 0 ? cfg.engine_workers : cfg.max_ctas));
     WorkItem w{};
     w.desc.scenario = static_cast<uint32_t>(op);
     w.desc.count = count;
     w.desc.compression_flags = compressed ? 1u : 0u;
     w.comm_size = world;
     w.udtype = static_cast<uint32_t>(dtype);
-    plan_call(exch.data(), cfg, w);
-    static const char *names[] = {"auto", "local", "eager", "nvls", "p2p", "p2p_oneshot", "ll", "staged", "wire"};
-    py::dict d;
-    d["algo"] = w.algo < 9 ? names[w.algo] : "?";
-    d["n_ctas"] = w.n_ctas;
-    d["use_mc"] = (w.flags & WF_USE_MC) != 0;
-    d["oneshot"] = (w.flags & WF_ONESHOT) != 0;
-    return d;
-  }, py::arg("op"), py::arg("count"), py::arg("dtype"), py::arg("world"), py::arg("max_eager_bytes") = 65536,
-        py::arg("max_ctas") = 128, py::arg("has_mc") = true, py::arg("nvls_min_ranks") = 3,
-        py::arg("oneshot_max_bytes") = 2u << 20, py::arg("compressed") = false, py::arg("stage_kb") = 1024, py::arg("ll_kb") = 256,
-        py::arg("ll_max_bytes") = 2 << 20, py::arg("ll_oneshot_max") = 32768, py::arg("staged_max_bytes") = 0,
-        py::arg("engine_mode") = false);
+    plan_call(exch.data(),
+              make_plan_cfg(cfg, has_mc, world, size_t{stage_kb} << 10, size_t{ll_kb} << 10, engine_mode ? workers : 0u), w);
+    return plan_dict(w);
+  }, py::arg("op"), py::arg("count"), py::arg("dtype"), py::arg("world"), py::kw_only(), py::arg("max_eager_bytes") = 64u << 10,
+        py::arg("eager_rx_buf_bytes") = 64u << 10, py::arg("has_mc") = true, py::arg("stage_kb") = 1024, py::arg("ll_kb") = 256,
+        py::arg("engine_mode") = false, py::arg("compressed") = false);
+  // how a live device plans a call: its exchange memory and plan_cfg(), without running the call
+  m.def("cuda_plan_call", [](ACCL &a, operation op, uint32_t count, dataType dtype, communicatorId comm_id) {
+    CCLO::Options o;
+    o.scenario = op;
+    o.count = count;
+    o.comm = comm_id;
+    o.arithcfg_addr = a.get_arithmetic_config_addr({dtype, dtype});
+    WorkItem w;
+    uint32_t err = 0;
+    if (!cuda_device(a)->build_work_item(o, make_call_desc(o), w, err)) throw std::invalid_argument("cuda_plan_call: error " + std::to_string(err));
+    return plan_dict(w);
+  }, py::arg("accl"), py::arg("op"), py::arg("count"), py::arg("dtype"), py::arg("comm_id") = 0);
   m.def("cuda_set_tuning", [](ACCL &a, const std::string &name, long value) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
-    if (!d->set_tuning(name, value)) throw std::invalid_argument("unknown tuning knob '" + name + "'");
+    if (!cuda_device(a)->set_tuning(name, value)) throw std::invalid_argument("unknown tuning knob '" + name + "'");
   });
-  m.def("cuda_get_tuning", [](ACCL &a, const std::string &name) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
-    return d->get_tuning(name);
-  });
+  m.def("cuda_get_tuning", [](ACCL &a, const std::string &name) { return cuda_device(a)->get_tuning(name); });
   m.def("cuda_drain", [](ACCL &a) {
     auto *d = dynamic_cast<CudaDevice *>(a.device());
     if (d) d->drain();
   }, py::call_guard<py::gil_scoped_release>());
   // zero-copy operands for memory that already lives in the heap (torch tensors from the heap pool)
   m.def("cuda_wrap_device", [](ACCL &a, uintptr_t dev_ptr, size_t n, dataType t) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     const size_t bytes = n * dtype_bytes(t);
     return std::unique_ptr<BaseBuffer>(new BaseBuffer(d->wrap_device(reinterpret_cast<void *>(dev_ptr), bytes), 0, bytes, t));
   });
   m.def("cuda_heap_range", [](ACCL &a) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     return std::make_pair(reinterpret_cast<uintptr_t>(d->heap().local()), d->heap().bytes());
   });
-  m.def("cuda_heap_pool_attach", [](ACCL &a) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
-    heap_pool_attach(d);
-  });
-  m.def("cuda_debug_state", [](ACCL &a) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
-    return d->debug_state();
-  });
+  m.def("cuda_heap_pool_attach", [](ACCL &a) { heap_pool_attach(cuda_device(a)); });
+  m.def("cuda_debug_state", [](ACCL &a) { return cuda_device(a)->debug_state(); });
   // out_shard[M/P, N] (heap buffer, bf16) = reduce_scatter_M( A[M,K] @ W[N,K]^T ), fused on tcgen05 + NVLink
   m.def("gemm_reduce_scatter", [](ACCL &a, uintptr_t a_ptr, uintptr_t w_ptr, BaseBuffer &out, uint32_t M, uint32_t N, uint32_t K,
                                   uintptr_t stream, int variant) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     GemmRsArgs g{reinterpret_cast<const void *>(a_ptr), reinterpret_cast<const void *>(w_ptr), out.address(), M, N, K, 0};
     g.variant = variant;
     g.out_f32 = out.type() == dataType::float32;
@@ -146,8 +115,7 @@ void bind_cuda(py::module_ &m) {
   // out = allreduce_sum(x + y): the kernel computes and then issues the collective itself (device API -> engine)
   m.def("vadd_allreduce", [](ACCL &a, BaseBuffer &x, BaseBuffer &y, BaseBuffer &tmp, BaseBuffer &out, uint32_t count,
                              uintptr_t status_dev_ptr, uintptr_t stream, uint32_t chunk_elems) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     cudaError_t e = launch_vadd_allreduce(*d, x.address(), y.address(), tmp.address(), out.address(), count, chunk_elems,
                                           static_cast<uint32_t>(a.get_communicator_addr(GLOBAL_COMM)),
                                           static_cast<uint32_t>(a.get_arithmetic_config_addr({dataType::float32, dataType::float32})),
@@ -158,53 +126,38 @@ void bind_cuda(py::module_ &m) {
   // the reference's vadd_put example: src + 1 pushed into stream `stream_id` of rank dst while computing
   m.def("vadd_put", [](ACCL &a, BaseBuffer &src, uint32_t count, uint32_t dst_rank, uint32_t stream_id, uintptr_t status_dev_ptr,
                        uintptr_t stream) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     cudaError_t e = launch_vadd_put(*d, src.address(), count, dst_rank, stream_id, reinterpret_cast<uint32_t *>(status_dev_ptr),
                                     reinterpret_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) throw std::runtime_error(std::string("vadd_put launch: ") + cudaGetErrorString(e));
   }, py::call_guard<py::gil_scoped_release>());
   m.def("stream_pull", [](ACCL &a, BaseBuffer &dst, uint32_t count, uint32_t stream_id, uintptr_t status_dev_ptr, uintptr_t stream) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     cudaError_t e = launch_stream_pull(*d, dst.address(), count, stream_id, reinterpret_cast<uint32_t *>(status_dev_ptr),
                                        reinterpret_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) throw std::runtime_error(std::string("stream_pull launch: ") + cudaGetErrorString(e));
   }, py::call_guard<py::gil_scoped_release>());
   m.def("stream_loopback", [](ACCL &a, BaseBuffer &scratch, uint32_t count, bool add_one, uintptr_t status_dev_ptr,
                               uintptr_t stream) {
-    auto *d = dynamic_cast<CudaDevice *>(a.device());
-    if (!d) throw std::runtime_error("not a CUDA backend");
+    CudaDevice *d = cuda_device(a);
     cudaError_t e = launch_loopback(*d, scratch.address(), count, add_one, reinterpret_cast<uint32_t *>(status_dev_ptr),
                                     reinterpret_cast<cudaStream_t>(stream));
     if (e != cudaSuccess) throw std::runtime_error(std::string("stream_loopback launch: ") + cudaGetErrorString(e));
   }, py::call_guard<py::gil_scoped_release>());
   m.def("cuda_probe", [](int device) { return probe_topology(device).describe(); });
   // N ranks in this process (threads), rank i on devices[i]
-  m.def("make_cuda_world", [](std::vector<int> devices, size_t heap_mb, bool multicast, int max_ctas, bool engine,
-                              int nvls_min_ranks, size_t oneshot_kb, int nvls_ops, const Extra &extra) {
+  m.def("make_cuda_world", [](std::vector<int> devices, const OptionMap &options) {
     std::vector<std::unique_ptr<ACCL>> out;
-    auto devs = make_local_world(devices, make_cfg(0, heap_mb, multicast, max_ctas, engine, nvls_min_ranks, oneshot_kb, nvls_ops, extra));
-    for (auto &d : devs) {
-      apply_extra(*d, extra);
-      out.emplace_back(new ACCL(std::move(d)));
-    }
+    for (auto &d : make_local_world(devices, config_from(options))) out.emplace_back(new ACCL(std::move(d)));
     return out;
-  }, py::arg("devices"), py::arg("heap_mb") = 256, py::arg("multicast") = true, py::arg("max_ctas") = 32,
-        py::arg("engine") = false, py::arg("nvls_min_ranks") = 3, py::arg("oneshot_kb") = 2048, py::arg("nvls_ops") = -1,
-        py::arg("extra") = Extra{}, py::call_guard<py::gil_scoped_release>());
+  }, py::arg("devices"), py::arg("options"), py::call_guard<py::gil_scoped_release>());
   // one rank per process; bootstrap over a private TCP rendezvous on addr:port
-  m.def("make_cuda_rank", [](int rank, int world, int device, const std::string &addr, int port, size_t heap_mb,
-                             bool multicast, int max_ctas, bool engine, int nvls_min_ranks, size_t oneshot_kb, int nvls_ops,
-                             const Extra &extra) {
+  m.def("make_cuda_rank", [](int rank, int world, int device, const std::string &addr, int port, const OptionMap &options) {
+    CudaConfig cfg = config_from(options);
+    cfg.device = device;
     auto oob = std::make_shared<TcpOob>(rank, world, addr, port);
-    auto cd = std::unique_ptr<CudaDevice>(
-        new CudaDevice(oob, make_cfg(device, heap_mb, multicast, max_ctas, engine, nvls_min_ranks, oneshot_kb, nvls_ops, extra)));
-    apply_extra(*cd, extra);
-    return std::unique_ptr<ACCL>(new ACCL(std::unique_ptr<CCLO>(std::move(cd))));
-  }, py::arg("rank"), py::arg("world_size"), py::arg("device"), py::arg("addr") = "127.0.0.1", py::arg("port") = 29637,
-        py::arg("heap_mb") = 1024, py::arg("multicast") = true, py::arg("max_ctas") = 32, py::arg("engine") = false,
-        py::arg("nvls_min_ranks") = 3, py::arg("oneshot_kb") = 2048, py::arg("nvls_ops") = -1, py::arg("extra") = Extra{},
+    return std::unique_ptr<ACCL>(new ACCL(std::unique_ptr<CCLO>(new CudaDevice(oob, cfg))));
+  }, py::arg("rank"), py::arg("world_size"), py::arg("device"), py::arg("addr"), py::arg("port"), py::arg("options"),
         py::call_guard<py::gil_scoped_release>());
 }
 

@@ -446,66 +446,100 @@ uint32_t CudaDevice::host_config(const CallDesc &d) {
   return COLLECTIVE_NOT_IMPLEMENTED;
 }
 
-PlanCfg CudaDevice::plan_cfg() const {
+// ------------------------------------------------------------------ options
+namespace {
+struct Option {
+  const char *name;
+  bool runtime; // may change after construction (set_tuning / get_tuning / ACCL_TUNE)
+  void (*set)(CudaConfig &c, long v, bool running);
+  long (*get)(const CudaConfig &c); // run-time options only
+};
+
+// options stored as they are given
+template <auto F> void put(CudaConfig &c, long v, bool) { c.*F = static_cast<std::decay_t<decltype(c.*F)>>(v); }
+template <auto F> long get(const CudaConfig &c) { return static_cast<long>(c.*F); }
+template <uint8_t Tune::*F> long get_tune(const CudaConfig &c) { return c.tune.*F; }
+
+const Option OPTIONS[] = {
+    {"heap_mb", false, [](CudaConfig &c, long v, bool) { c.heap_bytes = static_cast<size_t>(v) << 20; }, nullptr},
+    {"multicast", false, put<&CudaConfig::multicast>, nullptr},
+    {"engine", false, put<&CudaConfig::engine>, nullptr},
+    {"engine_workers", false, put<&CudaConfig::engine_workers>, nullptr},
+    {"engine_idle_us", false, put<&CudaConfig::engine_idle_us>, nullptr},
+    {"oneshot_kb", false, [](CudaConfig &c, long v, bool) { c.oneshot_max_bytes = static_cast<size_t>(v) << 10; }, nullptr},
+    {"nvls_ops", false, [](CudaConfig &c, long v, bool) { if (v >= 0) c.nvls_ops = static_cast<uint32_t>(v); }, nullptr}, // < 0: default
+    {"stage_kb", false, [](CudaConfig &c, long v, bool) { c.stage_bytes = static_cast<size_t>(v) << 10; }, nullptr},
+    {"ll_kb", false, [](CudaConfig &c, long v, bool) { c.ll_bytes = static_cast<size_t>(v) << 10; }, nullptr},
+    {"host_pipeline_chunk_kb", false, [](CudaConfig &c, long v, bool) { c.host_pipeline_chunk = static_cast<size_t>(v) << 10; }, nullptr},
+    // A live device keeps max_ctas below the sync channels of the engine and of the GEMM plugin (the two last ones);
+    // construction accepts up to all of them, and the benchmarks run with 128.
+    {"max_ctas", true, [](CudaConfig &c, long v, bool running) { c.max_ctas = static_cast<int>(running ? std::max(1l, std::min<long>(MAX_CH - 2, v)) : v); }, get<&CudaConfig::max_ctas>},
+    {"nvls_min_ranks", true, put<&CudaConfig::nvls_min_ranks>, get<&CudaConfig::nvls_min_ranks>},
+    {"nvls_ctas", true, put<&CudaConfig::nvls_ctas>, get<&CudaConfig::nvls_ctas>},
+    {"hybrid_16ths", true, [](CudaConfig &c, long v, bool) { c.tune.hybrid_16ths = static_cast<uint8_t>(std::max(0l, std::min(15l, v))); }, get_tune<&Tune::hybrid_16ths>},
+    {"nvls_unroll", true, [](CudaConfig &c, long v, bool) { c.tune.nvls_unroll = static_cast<uint8_t>(v == 2 || v == 8 || v == 16 ? v : 4); }, get_tune<&Tune::nvls_unroll>},
+    {"reduce_push", true, [](CudaConfig &c, long v, bool) { c.tune.reduce_push = static_cast<uint8_t>(v < 0 || v > 2 ? 0 : v); }, get_tune<&Tune::reduce_push>},
+    {"bcast_flags", true, [](CudaConfig &c, long v, bool) { c.tune.bcast_flags = static_cast<uint8_t>(v < 0 || v > 2 ? 0 : v); }, get_tune<&Tune::bcast_flags>},
+    {"split_phases", true, [](CudaConfig &c, long v, bool) { c.tune.split_phases = v ? 1 : 0; }, get_tune<&Tune::split_phases>},
+    {"ll_max_bytes", true, put<&CudaConfig::ll_max_bytes>, get<&CudaConfig::ll_max_bytes>},
+    {"ll_oneshot_max", true, put<&CudaConfig::ll_oneshot_max>, get<&CudaConfig::ll_oneshot_max>},
+    {"oneshot_max_bytes", true, put<&CudaConfig::oneshot_max_bytes>, get<&CudaConfig::oneshot_max_bytes>},
+    {"wire_min_bytes", true, put<&CudaConfig::wire_min_bytes>, get<&CudaConfig::wire_min_bytes>},
+    {"staged_max_bytes", true, put<&CudaConfig::staged_max_bytes>, get<&CudaConfig::staged_max_bytes>},
+    {"stream_loopback", true, put<&CudaConfig::stream_loopback>, get<&CudaConfig::stream_loopback>},
+};
+
+const Option *find_option(const std::string &name) {
+  for (const Option &o : OPTIONS) if (name == o.name) return &o;
+  return nullptr;
+}
+} // namespace
+
+bool set_option(CudaConfig &c, const std::string &name, long value, bool running) {
+  const Option *o = find_option(name);
+  if (!o || (running && !o->runtime)) return false;
+  o->set(c, value, running);
+  return true;
+}
+
+PlanCfg make_plan_cfg(const CudaConfig &cfg, bool has_mc, uint32_t heap_world, size_t stg_bytes, size_t ll_bytes,
+                      uint32_t engine_workers) {
   PlanCfg c;
   std::memset(&c, 0, sizeof(c));
-  c.max_ctas = static_cast<uint32_t>(cfg_.max_ctas);
-  if (engine_) c.max_ctas = std::min<uint32_t>(c.max_ctas, static_cast<uint32_t>(engine_->workers())); // channels == worker CTAs
-  c.nvls_min_ranks = static_cast<uint32_t>(cfg_.nvls_min_ranks);
-  c.has_mc = heap_->has_multicast() ? 1u : 0u;
-  c.heap_world = static_cast<uint32_t>(heap_->world());
-  c.oneshot_max_bytes = cfg_.oneshot_max_bytes;
-  c.nvls_ops = cfg_.nvls_ops;
-  c.nvls_ctas = static_cast<uint32_t>(cfg_.nvls_ctas);
-  c.stg_bytes = static_cast<uint32_t>(world_.stg_bytes);
-  c.ll_bytes = static_cast<uint32_t>(world_.ll_bytes);
-  c.ll_max_bytes = static_cast<uint32_t>(cfg_.ll_max_bytes);
-  c.ll_oneshot_max = static_cast<uint32_t>(cfg_.ll_oneshot_max);
-  c.wire_min_bytes = static_cast<uint32_t>(cfg_.wire_min_bytes);
-  c.staged_max_bytes = static_cast<uint32_t>(cfg_.staged_max_bytes);
-  c.engine_mode = engine_ ? 1u : 0u;
-  c.tune = cfg_.tune;
+  c.max_ctas = static_cast<uint32_t>(cfg.max_ctas);
+  if (engine_workers) c.max_ctas = std::min(c.max_ctas, engine_workers);
+  c.nvls_min_ranks = static_cast<uint32_t>(cfg.nvls_min_ranks);
+  c.has_mc = has_mc ? 1u : 0u;
+  c.heap_world = heap_world;
+  c.oneshot_max_bytes = cfg.oneshot_max_bytes;
+  c.nvls_ops = cfg.nvls_ops;
+  c.nvls_ctas = static_cast<uint32_t>(cfg.nvls_ctas);
+  c.stg_bytes = static_cast<uint32_t>(stg_bytes);
+  c.ll_bytes = static_cast<uint32_t>(ll_bytes);
+  c.ll_max_bytes = static_cast<uint32_t>(cfg.ll_max_bytes);
+  c.ll_oneshot_max = static_cast<uint32_t>(cfg.ll_oneshot_max);
+  c.wire_min_bytes = static_cast<uint32_t>(cfg.wire_min_bytes);
+  c.staged_max_bytes = static_cast<uint32_t>(cfg.staged_max_bytes);
+  c.engine_mode = engine_workers ? 1u : 0u;
+  c.tune = cfg.tune;
   return c;
+}
+
+PlanCfg CudaDevice::plan_cfg() const {
+  return make_plan_cfg(cfg_, heap_->has_multicast(), static_cast<uint32_t>(heap_->world()), world_.stg_bytes,
+                       world_.ll_bytes, engine_ ? static_cast<uint32_t>(engine_->workers()) : 0u);
 }
 
 bool CudaDevice::set_tuning(const std::string &name, long v) {
   std::lock_guard<std::mutex> lk(m_);
-  if (name == "hybrid_16ths") cfg_.tune.hybrid_16ths = static_cast<uint8_t>(std::max(0l, std::min(15l, v)));
-  else if (name == "nvls_unroll") cfg_.tune.nvls_unroll = static_cast<uint8_t>(v == 2 || v == 8 || v == 16 ? v : 4);
-  else if (name == "reduce_push") cfg_.tune.reduce_push = static_cast<uint8_t>(v < 0 || v > 2 ? 0 : v);
-  else if (name == "bcast_flags") cfg_.tune.bcast_flags = static_cast<uint8_t>(v < 0 || v > 2 ? 0 : v);
-  else if (name == "split_phases") cfg_.tune.split_phases = v ? 1 : 0;
-  else if (name == "nvls_ctas") cfg_.nvls_ctas = static_cast<int>(v);
-  else if (name == "nvls_min_ranks") cfg_.nvls_min_ranks = static_cast<int>(v);
-  else if (name == "max_ctas") cfg_.max_ctas = static_cast<int>(std::max(1l, std::min<long>(MAX_CH - 2, v)));
-  else if (name == "ll_max_bytes") cfg_.ll_max_bytes = static_cast<size_t>(v);
-  else if (name == "ll_oneshot_max") cfg_.ll_oneshot_max = static_cast<size_t>(v);
-  else if (name == "oneshot_max_bytes") cfg_.oneshot_max_bytes = static_cast<size_t>(v);
-  else if (name == "wire_min_bytes") cfg_.wire_min_bytes = static_cast<size_t>(v);
-  else if (name == "staged_max_bytes") cfg_.staged_max_bytes = static_cast<size_t>(v);
-  else if (name == "stream_loopback") strm_loopback_ = v != 0;
-  else return false;
-  return true;
+  return set_option(cfg_, name, v, true);
 }
 
 long CudaDevice::get_tuning(const std::string &name) const {
-  if (name == "hybrid_16ths") return cfg_.tune.hybrid_16ths;
-  if (name == "nvls_unroll") return cfg_.tune.nvls_unroll;
-  if (name == "reduce_push") return cfg_.tune.reduce_push;
-  if (name == "bcast_flags") return cfg_.tune.bcast_flags;
-  if (name == "split_phases") return cfg_.tune.split_phases;
-  if (name == "nvls_ctas") return cfg_.nvls_ctas;
-  if (name == "nvls_min_ranks") return cfg_.nvls_min_ranks;
-  if (name == "max_ctas") return cfg_.max_ctas;
-  if (name == "ll_max_bytes") return static_cast<long>(cfg_.ll_max_bytes);
-  if (name == "ll_oneshot_max") return static_cast<long>(cfg_.ll_oneshot_max);
-  if (name == "oneshot_max_bytes") return static_cast<long>(cfg_.oneshot_max_bytes);
-  if (name == "wire_min_bytes") return static_cast<long>(cfg_.wire_min_bytes);
-  if (name == "staged_max_bytes") return static_cast<long>(cfg_.staged_max_bytes);
-  if (name == "stream_loopback") return strm_loopback_ ? 1 : 0;
   if (name == "stage_bytes") return static_cast<long>(world_.stg_bytes);
   if (name == "ll_bytes") return static_cast<long>(world_.ll_bytes);
-  return -1;
+  const Option *o = find_option(name);
+  return o && o->runtime ? o->get(cfg_) : -1;
 }
 
 // ACCL_TUNE="name=value,name=value": experiment without rebuilding (must be identical on every rank)
@@ -592,7 +626,7 @@ ACCLRequest *CudaDevice::start(const Options &options) {
   uint32_t push_rank = world_.rank;
   bool put_only = false;
   // stream id (TDEST) of a streamed result: the tag of stream_put / recv-to-stream when it is a user id
-  const uint32_t res_strm_id = (!strm_loopback_ && options.tag >= STREAM_ID_MIN && options.tag <= STREAM_ID_MAX) ? options.tag : 0;
+  const uint32_t res_strm_id = (!cfg_.stream_loopback && options.tag >= STREAM_ID_MIN && options.tag <= STREAM_ID_MAX) ? options.tag : 0;
   const bool lowered = op0_strm || res_strm;
   if (lowered && engine_) drain_locked(); // the lowering kernels below are direct launches: they take over the engine's channels
   if (op0_strm || res_strm) {

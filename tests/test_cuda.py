@@ -493,3 +493,41 @@ def test_stream_ids_do_not_interleave():
         assert torch.equal(d1.dev.cpu(), data(n, prv, salt=1) + 1.0)
         a.barrier()
     run(2, fn, EAGER)
+
+
+# run-time knob: (value set, value read back), in range and out of range
+TUNING = {
+    "hybrid_16ths": [(3, 3), (99, 15), (-1, 0)],
+    "nvls_unroll": [(8, 8), (16, 16), (3, 4), (0, 4)],
+    "reduce_push": [(2, 2), (3, 0), (-1, 0)],
+    "bcast_flags": [(1, 1), (5, 0), (-2, 0)],
+    "split_phases": [(1, 1), (7, 1), (0, 0)],
+    "nvls_ctas": [(16, 16), (1 << 20, 1 << 20)],
+    "nvls_min_ranks": [(2, 2), (99, 99)],
+    "max_ctas": [(64, 64), (126, 126), (127, 126), (1000, 126), (0, 1), (-5, 1)],
+    "ll_max_bytes": [(1 << 20, 1 << 20), (1 << 40, 1 << 40), (-1, -1)],
+    "ll_oneshot_max": [(8 << 10, 8 << 10), (1 << 40, 1 << 40)],
+    "oneshot_max_bytes": [(1 << 20, 1 << 20), (1 << 40, 1 << 40)],
+    "wire_min_bytes": [(0, 0), (1 << 40, 1 << 40)],
+    "staged_max_bytes": [(1 << 20, 1 << 20), (1 << 40, 1 << 40)],
+    "stream_loopback": [(0, 0), (5, 1), (1, 1)],
+}
+
+
+def test_set_tuning_clamps_and_get_tuning_reads_back():
+    """Every run-time knob takes an in-range value as it is and clamps (or stores) an out-of-range one; the options
+    fixed at construction are refused by set_tuning and unknown to get_tuning; max_ctas=128 at construction stays 128."""
+    def fn(a, r, w):
+        assert a.get_tuning("max_ctas") == 128
+        for name, pairs in TUNING.items():
+            for value, want in pairs:
+                a.set_tuning(name, value)
+                assert a.get_tuning(name) == want, (name, value)
+        for name in ("heap_mb", "multicast", "engine", "engine_workers", "engine_idle_us", "oneshot_kb", "nvls_ops",
+                     "stage_kb", "ll_kb", "host_pipeline_chunk_kb", "stage_bytes", "ll_bytes", "no_such_knob"):
+            with pytest.raises(ValueError):
+                a.set_tuning(name, 1)
+        for name in ("engine_workers", "stage_kb", "oneshot_kb", "no_such_knob"):
+            assert a.get_tuning(name) == -1, name
+        assert a.get_tuning("stage_bytes") > 0 and a.get_tuning("ll_bytes") > 0
+    A.run_cuda_ranks([0], fn, EAGER, heap_mb=64, max_ctas=128)

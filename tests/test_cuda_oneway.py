@@ -45,11 +45,9 @@ def run(world, fn, **kw):
     return A.run_cuda_ranks(devices(world), fn, ONEWAY, **cfg)
 
 
-def algo(a, op, count, dtype=A.DataType.float32, world=2):
-    """what the planner picks on this backend configuration (pure function, same on every rank)"""
-    return A._C.cuda_plan(op, count, dtype, world, max_eager_bytes=4 << 20, max_ctas=16, stage_kb=a.get_tuning("stage_bytes") >> 10,
-                          ll_kb=a.get_tuning("ll_bytes") >> 10, ll_max_bytes=a.get_tuning("ll_max_bytes"),
-                          ll_oneshot_max=a.get_tuning("ll_oneshot_max"), staged_max_bytes=a.get_tuning("staged_max_bytes"))
+def algo(a, op, count, dtype=A.DataType.float32):
+    """what the planner picks for this call on this device (same on every rank)"""
+    return A._C.cuda_plan_call(a.impl, op, count, dtype)
 
 
 # counts (fp32): 1 elem, odd tiny, 1 KiB, LL one-hop limit, two-hop LL, LL/staged crossover, staged, odd staged
@@ -70,7 +68,7 @@ def test_allreduce_sizes(world, func):
             torch.cuda.current_stream().synchronize()
             assert close(d.dev, ref_reduce(w, n, func, salt=n), 1e-5, 1e-4), f"allreduce n={n} rank {r}"
             if r == 0:
-                p = algo(a, A._C.Operation.allreduce, n, world=w)
+                p = algo(a, A._C.Operation.allreduce, n)
                 seen.add((p["algo"], p["oneshot"]))
     run(world, fn)
     assert ("ll", True) in seen and ("staged", False) in seen, seen

@@ -220,7 +220,8 @@ def test_one_shot_or_two_shot_is_the_planners_decision(cfg, max_eager):
     world = 4
     Op = A._C.Operation
     for count in (256, 8192, 65536, 262144):
-        p = A._C.cuda_plan(Op.allreduce, count, A.DataType.float32, world, max_eager_bytes=max_eager, ll_kb=2048)
+        p = A._C.cuda_plan(Op.allreduce, count, A.DataType.float32, world, max_eager_bytes=max_eager,
+                           eager_rx_buf_bytes=64 << 10, max_ctas=128, stage_kb=1024, ll_kb=2048)
         want_one_shot = p["algo"] in ("p2p_oneshot", "eager") or (p["algo"] in ("ll", "staged") and p["oneshot"])
 
         def fn(a, r, w, count=count):

@@ -11,8 +11,13 @@ Op = A._C.Operation
 F32 = DataType.float32
 
 
+# the configuration these tests were written against: 128 channels, 1 MiB staging / 256 KiB LL regions, 64 KiB eager
+# limits; every other option at its CudaConfig default
+PINNED = dict(max_ctas=128, stage_kb=1024, ll_kb=256, max_eager_bytes=64 << 10, eager_rx_buf_bytes=64 << 10)
+
+
 def plan(op, nbytes, world=8, dtype=F32, esz=4, **kw):
-    return A._C.cuda_plan(op, nbytes // esz, dtype, world, **kw)
+    return A._C.cuda_plan(op, nbytes // esz, dtype, world, **{**PINNED, **kw})
 
 
 ONE_WAY = ("eager", "ll", "staged")  # protocols without a meeting: slot ring, flag-in-data, payload + flag
@@ -111,8 +116,9 @@ COLLECTIVES = [Op.allreduce, Op.allgather, Op.reduce_scatter, Op.bcast, Op.scatt
        has_mc=st.booleans(), ll_kb=st.sampled_from([0, 64, 256, 2048]), stage_kb=st.sampled_from([0, 1024]),
        staged_max=st.sampled_from([0, 1 << 20]), engine_mode=st.booleans(), compressed=st.booleans())
 def test_plans_are_executable(op, count, world, max_eager, max_ctas, has_mc, ll_kb, stage_kb, staged_max, engine_mode, compressed):
-    p = A._C.cuda_plan(op, count, F32, world, max_eager_bytes=max_eager, max_ctas=max_ctas, has_mc=has_mc, ll_kb=ll_kb,
-                       stage_kb=stage_kb, staged_max_bytes=staged_max, engine_mode=engine_mode, compressed=compressed)
+    p = A._C.cuda_plan(op, count, F32, world, max_eager_bytes=max_eager, eager_rx_buf_bytes=64 << 10, max_ctas=max_ctas,
+                       has_mc=has_mc, ll_kb=ll_kb, stage_kb=stage_kb, staged_max_bytes=staged_max, engine_mode=engine_mode,
+                       compressed=compressed)
     nbytes = count * 4
     assert p["algo"] in ("eager", "nvls", "p2p", "p2p_oneshot", "ll", "staged", "wire")
     assert 1 <= p["n_ctas"] <= min(max(max_ctas, 1), 128)                     # never more channels than sync pads / the cap
@@ -144,3 +150,23 @@ def test_channel_count_grows_with_the_message_within_one_protocol(op, world, lo)
     b = plan(op, lo * 8, world=world, max_eager_bytes=4 << 20, ll_kb=2048)
     if a["algo"] == b["algo"] and a["oneshot"] == b["oneshot"]:
         assert b["n_ctas"] >= a["n_ctas"], (a, b)
+
+
+def test_options_default_to_the_device_configuration():
+    """No option given plans as a device built with every CudaConfig default; unknown names are refused."""
+    nvls_ops = (1 << int(Op.allreduce)) | (1 << int(Op.bcast)) | (1 << int(Op.reduce))
+    defaults = dict(heap_mb=1024, multicast=1, engine=0, engine_workers=0, engine_idle_us=1000, oneshot_kb=2048,
+                    nvls_ops=nvls_ops, host_pipeline_chunk_kb=16 << 10, max_ctas=32, nvls_min_ranks=3, nvls_ctas=32,
+                    hybrid_16ths=0, nvls_unroll=4, reduce_push=0, bcast_flags=0, split_phases=0, ll_max_bytes=2 << 20,
+                    ll_oneshot_max=32 << 10, oneshot_max_bytes=2 << 20, wire_min_bytes=256 << 10, staged_max_bytes=0,
+                    stream_loopback=1)
+    geometry = dict(max_eager_bytes=4 << 20, eager_rx_buf_bytes=64 << 10, stage_kb=1024, ll_kb=256)
+    for op in COLLECTIVES + [Op.send]:
+        for nbytes in (1024, 64 << 10, 1 << 20, 16 << 20, 256 << 20):
+            for world in (2, 4, 8):
+                for engine_mode in (False, True):
+                    call = (op, nbytes // 4, F32, world)
+                    assert (A._C.cuda_plan(*call, engine_mode=engine_mode, **geometry) ==
+                            A._C.cuda_plan(*call, engine_mode=engine_mode, **geometry, **defaults)), (call, engine_mode)
+    with pytest.raises(ValueError, match="unknown CUDA backend option 'no_such_knob'"):
+        A._C.cuda_plan(Op.allreduce, 1024, F32, 8, **geometry, no_such_knob=1)
